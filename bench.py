@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                      (our CUDA path)
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference [--workload embed|retrieval|train] (the reference on the host cores)
+    python bench.py ... --dump-outputs DIR                             (+ the last timed step's embeddings, DIR/*.npy)
 
 Primary metric (BASELINE.json): embeddings/sec @256x128 -- one "step" = one pass of the eval embedding path (trunk ->
 global average pool -> BatchNorm1d, modelling/bases.py:169-177) over one batch of 256 synthetic 256x128 crops per GPU,
@@ -147,6 +148,23 @@ def max_over_ranks(v, world, dev):
     return float(t.item())
 
 
+DUMP_BYTES = 63 << 20  # the arrays of --dump-outputs; the row lists of a sampled output fit in the rest of 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """`--dump-outputs`: each array as out_dir/<name>.npy in float32.  If they exceed DUMP_BYTES in all, each keeps a
+    fixed, seeded sample of its rows (the same rows in every run), listed in out_dir/<name>_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            rows = np.sort(np.random.default_rng(0).choice(len(a), max(1, len(a) * DUMP_BYTES // total), replace=False))
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def timed_steps(step_fn, steps, warmup, world, finish_fn=None):
     """W warm-ups, then EXACTLY `steps` steps (+ `finish_fn`, the one collective after extraction) between
     barrier + synchronize; device time via CUDA events on the launching stream, max over ranks."""
@@ -218,6 +236,9 @@ def run_embed(args, world, rank, local):
     finish()
     with clk.window():
         ms = timed_steps(step, steps, 0, world, finish)
+    if args.dump_outputs and rank == 0:  # before the e2e runs below reuse local_emb
+        emb = gathered[:, steps - 1].reshape(world * BATCH, 2048) if world > 1 else local_emb[steps - 1]
+        dump_outputs(args.dump_outputs, {"emb": emb, "global_feat": graphs[(steps - 1) % n_rot].out["global_feat"]})
     launches = (graphs[0].launches + 1) * steps
     value = world * BATCH * steps / (ms / 1e3)
 
@@ -870,7 +891,14 @@ def main():
     ap.add_argument("--train-size", default="256x128", help="HxW of the training crops (config 4: 320x320)")
     ap.add_argument("--train-pk", default="16x16", help="ids x instances per GPU (config 4: 32x4)")
     ap.add_argument("--no-secondary", action="store_true", help="skip the nested metrics and the CPU baselines")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (emb, global_feat) as DIR/<name>.npy "
+                         "(float32); the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "embed"):
+        ap.error("--dump-outputs records the embed workload of --impl ours")
     args.warmup = max(args.warmup, 3)
     world, rank, local = dist_env()
 

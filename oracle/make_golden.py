@@ -1,7 +1,8 @@
 """TEST INFRASTRUCTURE ONLY -- generates tests/golden/*.npz by running the UNMODIFIED
 reference (/root/reference, through oracle/ref_import.py) on seeded synthetic inputs.
 
-    python -m oracle.make_golden [--only loss,retrieval,trunk,trunk_train,trunk_autocast,masks,centroids,market]
+    python -m oracle.make_golden [--only loss,retrieval,trunk,trunk_train,trunk_autocast,masks,centroids,market,...]
+    python -m oracle.make_golden --only ref_cuda_autocast      (on a CUDA device: the reference at the bench shapes)
 
 The reference has no tests and no golden vectors of its own (SURVEY.md section 4); these
 files are what pins the oracle restatement (oracle/ctl_oracle.py) and, through it, the
@@ -357,9 +358,158 @@ def gen_trunk_autocast(ref):
     np.savez_compressed(os.path.join(GOLD, "trunk_autocast.npz"), **out)
 
 
+TRIPLET_VARIANTS = ((None, "euclidean"), (0.3, "cosine"), (None, "cosine"))
+TRIPLET_GRAD_ELEMS = np.sort(np.random.default_rng(0).choice(40 * 384, 2048, replace=False))  # of the flattened gradient
+
+
+def triplet_variant_batch():
+    feats, labels, is_real = O.synth_batch(10, 4, 384, 100, seed=4, pad_fraction=0.2)
+    return feats * 0.3 + 0.05, labels, is_real
+
+
+def gen_triplet_variants(ref):
+    """The reference's own TripletLoss (losses/triplet_loss.py) with a soft margin and with cosine distances: loss value
+    and a fixed sample of the input gradient on one batch."""
+    feats, labels, _ = triplet_variant_batch()
+    out = {"in_checksum": checksum(feats)}
+    for margin, dist in TRIPLET_VARIANTS:
+        fr = feats.clone().requires_grad_(True)
+        loss, _, _ = ref.triplet_loss.TripletLoss(margin, dist)(fr, labels)
+        loss.backward()
+        out[f"{dist}_{margin}_loss"] = loss.item()
+        out[f"{dist}_{margin}_grad"] = fr.grad.flatten()[TRIPLET_GRAD_ELEMS].numpy()
+        out[f"{dist}_{margin}_grad_absmax"] = float(fr.grad.abs().max())
+    np.savez_compressed(os.path.join(GOLD, "triplet_variants.npz"), **out)
+    print("triplet variants done")
+
+
+ERASE_SHAPE, ERASE_SEEDS = (32, 20), 5
+ERASE_MEAN, ERASE_STD = (0.485, 0.456, 0.406), (0.229, 0.224, 0.225)
+
+
+def erase_input():
+    """One uint8 HWC image and its normalised CHW tensor (ToTensor + Normalize)."""
+    H, W = ERASE_SHAPE
+    img = torch.from_numpy(np.random.default_rng(1).integers(0, 256, (1, H, W, 3), dtype=np.uint8))
+    norm = (img[0].permute(2, 0, 1).float() / 255.0 - torch.tensor(ERASE_MEAN)[:, None, None]) / torch.tensor(ERASE_STD)[:, None, None]
+    return img, norm
+
+
+def gen_random_erasing(ref):
+    """The reference's own RandomErasing (datasets/transforms/random_erasing.py) on one normalised image, driven by
+    random.seed(s) for s in range(ERASE_SEEDS)."""
+    import importlib.util
+    import random
+
+    from oracle.ref_import import REFERENCE_ROOT
+
+    spec = importlib.util.spec_from_file_location(
+        "ref_random_erasing", os.path.join(REFERENCE_ROOT, "datasets", "transforms", "random_erasing.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    img, norm = erase_input()
+    outs = []
+    for seed in range(ERASE_SEEDS):
+        random.seed(seed)
+        outs.append(mod.RandomErasing(probability=1.0, mean=ERASE_MEAN)(norm.clone()).numpy())
+    np.savez_compressed(os.path.join(GOLD, "random_erasing.npz"), in_checksum=checksum(img), erased=np.stack(outs))
+    print("random erasing done")
+
+
+# The reference's trunk on a CUDA device under fp16 autocast at the bench shapes (tests/test_reference_autocast_gpu.py).
+# Whole outputs would not fit a small fixture, so every image is kept on a fixed sample of feature channels, and every
+# parameter gradient as a strided sample (grad_sample, in float16 over its largest magnitude: the test takes cosines of
+# it) next to the full tensor's norm and its fp16-vs-fp32 cosine.  The autocast features are fp16 values: stored exactly.
+AUTOCAST_EVAL_CASES = (("r50", False, (256, 128), 256), ("ibn", True, (320, 320), 128))
+AUTOCAST_TRAIN_CASES = (("r50 cfg2", False, (256, 128), 16, 16), ("ibn cfg4/gpu", True, (320, 320), 32, 4))
+AUTOCAST_FEAT_COLS = np.sort(np.random.default_rng(0).choice(2048, 32, replace=False))
+AUTOCAST_GRAD_SAMPLE = 128
+AUTOCAST_LOSS_SCALE = 1024.0
+
+
+def autocast_eval_input(ibn, hw, bs):
+    return O.make_trunk_state(seed=7, ibn=ibn), torch.randn(bs, 3, *hw, generator=torch.Generator().manual_seed(77))
+
+
+def autocast_train_input(ibn, hw, n):
+    gen = torch.Generator().manual_seed(5)
+    x = torch.randn(n, 3, *hw, generator=gen)
+    return O.make_trunk_state(seed=17, ibn=ibn), x, torch.randn(n, 2048, generator=gen) * 1e-3
+
+
+def golden_name(tag):
+    return tag.split()[0]
+
+
+def _ref_base_cuda(ref, ibn, sd):
+    cfg = default_cfg(ref)
+    cfg.MODEL.NAME = "resnet50_ibn_a" if ibn else "resnet50"
+    base = ref.baseline.Baseline(cfg)
+    base.base.load_state_dict(sd, strict=True)
+    return base.cuda()
+
+
+def gen_ref_cuda_autocast(ref):
+    """Needs a CUDA device.  Eval: global features of the eval trunk under torch.autocast(float16) and in fp32.  Train: one
+    train-mode step of sum(feat * dfeat) * AUTOCAST_LOSS_SCALE under autocast (features, unscaled gradients) and the
+    gradients of the same module in fp32."""
+    cols = torch.from_numpy(AUTOCAST_FEAT_COLS)
+    out = {"cols": AUTOCAST_FEAT_COLS}
+    for tag, ibn, hw, bs in AUTOCAST_EVAL_CASES:
+        sd, x = autocast_eval_input(ibn, hw, bs)
+        base = _ref_base_cuda(ref, ibn, sd).eval()
+        with torch.no_grad():
+            _, f32 = base(x.cuda())
+            with torch.autocast("cuda", dtype=torch.float16):
+                _, amp = base(x.cuda())
+        f32, amp = f32.float().cpu(), amp.float().cpu()
+        scale = float(f32.abs().max())
+        out[f"{tag}_in_checksum"] = checksum(x)
+        out[f"{tag}_scale"] = scale
+        out[f"{tag}_amp_vs_fp32"] = float((amp - f32).abs().max()) / scale
+        out[f"{tag}_feat_amp"] = amp[:, cols].half().numpy()
+        # fp32 features as their (small) distance to the autocast ones: fp16 keeps it to < 1e-6 of the feature scale
+        out[f"{tag}_feat_fp32_minus_amp"] = (f32 - amp)[:, cols].half().numpy()
+        print(f"ref cuda autocast eval {tag}: autocast vs fp32 {out[f'{tag}_amp_vs_fp32']:.3e}")
+        del base
+    np.savez_compressed(os.path.join(GOLD, "ref_cuda_autocast_eval.npz"), **out)
+    for tag, ibn, hw, P, K in AUTOCAST_TRAIN_CASES:
+        sd, x, dfeat = autocast_train_input(ibn, hw, P * K)
+        x, dfeat_d = x.cuda(), dfeat.cuda()
+        base = _ref_base_cuda(ref, ibn, sd).train()
+        with torch.autocast("cuda", dtype=torch.float16):
+            _, rfeat = base(x)
+        ((rfeat.float() * dfeat_d).sum() * AUTOCAST_LOSS_SCALE).backward()
+        rgrads = {k: (p.grad / AUTOCAST_LOSS_SCALE).cpu() for k, p in base.base.named_parameters() if p.grad is not None}
+        rfeat = rfeat.detach().float().cpu()
+        base.zero_grad(set_to_none=True)
+        base.base.load_state_dict(sd, strict=True)  # the first pass moved the running statistics
+        _, rfeat32 = base(x)
+        (rfeat32 * dfeat_d).sum().backward()
+        rgrads32 = {k: p.grad.cpu() for k, p in base.base.named_parameters() if p.grad is not None}
+        del base, rfeat32
+        torch.cuda.empty_cache()
+        keys = list(rgrads)
+        amp64, f64 = [rgrads[k].double() for k in keys], [rgrads32[k].double() for k in keys]
+        out = {"cols": AUTOCAST_FEAT_COLS, "in_checksum": checksum(torch.cat((x.cpu().flatten(), dfeat.flatten()))),
+               "feat_scale": float(rfeat.abs().max()), "feat_amp": rfeat[:, cols].half().numpy(), "keys": np.array(keys),
+               "norm_amp": np.array([float(a.norm()) for a in amp64]), "norm_fp32": np.array([float(b.norm()) for b in f64]),
+               "cos_amp_fp32": np.array([float((a * b).sum() / (a.norm() * b.norm() + 1e-300)) for a, b in zip(amp64, f64)])}
+        for name, grads in (("grad_amp", rgrads), ("grad_fp32", rgrads32)):
+            rows = np.zeros((len(keys), AUTOCAST_GRAD_SAMPLE), dtype=np.float16)  # row i: the sample of keys[i], zero-padded
+            for i, k in enumerate(keys):
+                s = grad_sample(grads[k], AUTOCAST_GRAD_SAMPLE)[:-2]
+                rows[i, :len(s)] = s / max(float(np.abs(s).max()), 1e-300)
+            out[name] = rows
+        np.savez_compressed(os.path.join(GOLD, f"ref_cuda_autocast_train_{golden_name(tag)}.npz"), **out)
+        print(f"ref cuda autocast train {tag}: {len(keys)} gradients, worst autocast-vs-fp32 cosine "
+              f"{out['cos_amp_fp32'].min():.4f}")
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--only", default="loss,loss_variants,masks,retrieval,centroids,trunk,trunk_train,trunk_autocast,market")
+    ap.add_argument("--only", default="loss,loss_variants,masks,retrieval,centroids,trunk,trunk_train,trunk_autocast,market,"
+                                      "triplet_variants,random_erasing")
     args = ap.parse_args()
     only = set(args.only.split(","))
     os.makedirs(GOLD, exist_ok=True)
@@ -386,6 +536,12 @@ def main():
     if "market" in only:
         # BASELINE config 3 shape; the reference's per-query python loop takes ~80 s here
         gen_retrieval(ref, "market", 3368, 15913, 751, 3.0, 0, store_dist=False)
+    if "triplet_variants" in only:
+        gen_triplet_variants(ref)
+    if "random_erasing" in only:
+        gen_random_erasing(ref)
+    if "ref_cuda_autocast" in only:  # needs a CUDA device; not in the default list
+        gen_ref_cuda_autocast(ref)
 
 
 if __name__ == "__main__":

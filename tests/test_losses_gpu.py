@@ -153,13 +153,14 @@ def test_centroids_match_reference_golden():
 def test_triplet_loss_soft_margin_and_cosine_variants(margin, dist):
     """TripletLoss(margin=None) (nn.SoftMarginLoss on dist_an - dist_ap) and dist_func='cosine'
     (losses/triplet_loss.py:44-65,127-137,157-158): value, mined distances and the gradient (through the row normalisation
-    for cosine) against autograd through the float64 oracle restatement, and against the reference's own class when its
-    vendored copy is on the box."""
+    for cosine) against autograd through the float64 oracle restatement, and against the reference's own class
+    (tests/golden/triplet_variants.npz, oracle/make_golden.py:gen_triplet_variants)."""
     from ctl_b200.losses.triplet_loss import TripletLoss
-    from oracle import ref_import
+    from oracle.make_golden import TRIPLET_GRAD_ELEMS, triplet_variant_batch
 
-    feats, labels, is_real = O.synth_batch(10, 4, 384, 100, seed=4, pad_fraction=0.2)
-    feats = feats * 0.3 + 0.05
+    feats, labels, is_real = triplet_variant_batch()
+    g = load_golden("triplet_variants.npz")
+    _close(checksum(feats), g["in_checksum"], 1e-12)
     for mask in (None, is_real):
         fo = feats.double().requires_grad_(True)
         lo, apo, ano = O.triplet_loss(fo, labels, margin, mask=mask, dist_func=dist)
@@ -171,13 +172,9 @@ def test_triplet_loss_soft_margin_and_cosine_variants(margin, dist):
         _close(apg.cpu().numpy(), apo.detach().numpy(), RTOL, 1e-6)
         _close(ang.cpu().numpy(), ano.detach().numpy(), RTOL, 1e-6)
         _close(fg.grad.cpu().numpy(), fo.grad.numpy(), RTOL, 1e-4 * float(fo.grad.abs().max()))
-    if ref_import.reference_available():
-        ref = ref_import.load_reference()
-        fr = feats.clone().requires_grad_(True)
-        lr, apr, anr = ref.triplet_loss.TripletLoss(margin, dist)(fr, labels)
-        lr.backward()
-        fg = feats.cuda().requires_grad_(True)
-        lg, apg, ang = TripletLoss(margin, dist)(fg, labels.cuda())
-        lg.backward()
-        _close(lg.item(), lr.item(), 2e-4)
-        _close(fg.grad.cpu().numpy(), fr.grad.numpy(), 2e-4, 2e-4 * float(fr.grad.abs().max()))
+    fg = feats.cuda().requires_grad_(True)
+    lg, apg, ang = TripletLoss(margin, dist)(fg, labels.cuda())
+    lg.backward()
+    _close(lg.item(), float(g[f"{dist}_{margin}_loss"]), 2e-4)
+    _close(fg.grad.cpu().flatten()[TRIPLET_GRAD_ELEMS].numpy(), g[f"{dist}_{margin}_grad"], 2e-4,
+           2e-4 * float(g[f"{dist}_{margin}_grad_absmax"]))
