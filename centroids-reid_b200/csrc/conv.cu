@@ -1715,8 +1715,14 @@ static int finish_and_launch(ConvKernelParams& p, int n, int Ho, int Wo, int cou
   return launch_conv<64>(p, st);
 }
 
+// rows (columns) of a side of `size` pixels whose index has parity `parity`: the extent of a stride-2 parity view
+static inline int parity_extent(int size, int parity) { return (size - parity + 1) / 2; }
+
 // A tensor maps of one NHWC source [n, h, w, cin] read at `stride`: stride 1 -> map 0..3 identical; stride 2 -> the four
-// parity views (view (ph, pw) holds input pixels (2i + ph, 2j + pw)), so every box is a dense stride-1 box.
+// parity views (view (ph, pw) holds input pixels (2i + ph, 2j + pw)), so every box is a dense stride-1 box.  Each view
+// has its own extent parity_extent(h, ph) x parity_extent(w, pw): on an odd side the odd view is one pixel shorter, and
+// the TMA zero-fill past its end is the convolution's zero padding.  A view that is empty (h == 1 or w == 1) gets a copy
+// of view (0, 0) so that every descriptor is valid; the caller issues no tap on it.
 static int encode_source(CUtensorMap* maps, int count, const void* x, int n, int h, int w, int cin, int stride, int TH,
                          int TW) {
   int rc;
@@ -1731,10 +1737,15 @@ static int encode_source(CUtensorMap* maps, int count, const void* x, int n, int
         return rc;
     return 0;
   }
-  const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)(w / 2), (uint64_t)(h / 2), (uint64_t)n};
   const uint64_t strd[4] = {2, (uint64_t)cin * 4, (uint64_t)w * cin * 4, (uint64_t)h * w * cin * 2};
   for (int v = 0; v < count; ++v) {
     const int ph = v >> 1, pw = v & 1;
+    const int vh = parity_extent(h, ph), vw = parity_extent(w, pw);
+    if (vh == 0 || vw == 0) {
+      maps[v] = maps[0];
+      continue;
+    }
+    const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)vw, (uint64_t)vh, (uint64_t)n};
     if ((rc = encode_tensor_map(&maps[v], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, 4, xb + ((size_t)ph * w + pw) * cin, dims,
                                 strd, abox, CU_TENSOR_MAP_SWIZZLE_128B)))
       return rc;
@@ -1757,7 +1768,6 @@ int ctl_conv2d_nhwc_f16(const void* x, int32_t n, int32_t h, int32_t w, int32_t 
   CTL_CHECK_ARG(cout <= 2048, "Cout=%d exceeds 2048 (bias staging)", cout);
   CTL_CHECK_ARG((ksize == 1 || ksize == 3) && (stride == 1 || stride == 2), "only 1x1 / 3x3, stride 1 / 2");
   CTL_CHECK_ARG(relu_from % 32 == 0, "relu_from=%d must be a multiple of 32", relu_from);
-  CTL_CHECK_ARG(stride == 1 || (h % 2 == 0 && w % 2 == 0), "stride 2 needs even H, W (got %dx%d)", h, w);
   int rc = ctl_device_check();
   if (rc) return rc;
   const int pad = ksize == 3 ? 1 : 0;
@@ -1772,20 +1782,22 @@ int ctl_conv2d_nhwc_f16(const void* x, int32_t n, int32_t h, int32_t w, int32_t 
   p.tiles_h = (Ho + p.TH - 1) / p.TH;
   p.tiles_w = (Wo + p.TW - 1) / p.TW;
   if ((rc = encode_source(p.a_map, 4, x, n, h, w, cin, stride, p.TH, p.TW))) return rc;
-  p.n_taps = ksize * ksize;
-  p.k_blocks = p.n_taps * (cin / 64);
+  p.n_taps = 0;
   for (int r = 0; r < ksize; ++r)
     for (int s = 0; s < ksize; ++s) {
       if (stride == 1) {
-        p.taps[r * ksize + s] = ConvTap{0, r - pad, s - pad, (r * ksize + s) * cin, cin / 64};
+        p.taps[p.n_taps++] = ConvTap{0, r - pad, s - pad, (r * ksize + s) * cin, cin / 64};
       } else {
         // input row 2*ho + r - pad = 2*(ho + dh) + ph
         const int ar = r - pad, as = s - pad;
         const int ph = ((ar % 2) + 2) % 2, pw = ((as % 2) + 2) % 2;
         const int dh = (ar - ph) / 2, dw = (as - pw) / 2;
-        p.taps[r * ksize + s] = ConvTap{ph * 2 + pw, dh, dw, (r * ksize + s) * cin, cin / 64};
+        // a tap on an empty parity view reads only padding: it adds exactly zero, so it is not issued
+        if (parity_extent(h, ph) == 0 || parity_extent(w, pw) == 0) continue;
+        p.taps[p.n_taps++] = ConvTap{ph * 2 + pw, dh, dw, (r * ksize + s) * cin, cin / 64};
       }
     }
+  p.k_blocks = p.n_taps * (cin / 64);
   return finish_and_launch(p, n, Ho, Wo, cout, ksize * ksize * cin, weight, bias, residual, out, relu, relu_from,
                            (cudaStream_t)stream);
 }

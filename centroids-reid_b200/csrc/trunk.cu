@@ -12,6 +12,7 @@
 #include <math.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <unordered_map>
 #include <vector>
@@ -314,15 +315,30 @@ int ctl_weights_pack(ctl_trunk* h, const ctl_named_tensor* tensors, int32_t n_te
   return 0;
 }
 
-static size_t trunk_act_bytes(int n, int hgt, int wid) {
-  // largest activation of the trunk: the stem's conv output [n, H/2, W/2, 64] == layer1's output [n, H/4, W/4, 256]
-  const size_t h2 = (hgt + 6 - 7) / 2 + 1, w2 = (wid + 6 - 7) / 2 + 1;
-  return ((size_t)n * h2 * w2 * 64 * 2 + 255) & ~(size_t)255;
+// Bytes of one of the five activation buffers of ctl_embed_forward: the largest activation of the trunk, found by a dry
+// walk of the layer shapes with the forward's own ceil formulas.  With even sides that is the stem's conv output
+// [n, H/2, W/2, 64] (== layer1's output [n, H/4, W/4, 256]).  When the stem output has an odd side the max-pool rounds
+// up and layer1's output is the larger one; at tiny inputs (8x8) a 1-pixel map of 1024 or 2048 channels is.
+static size_t trunk_act_bytes(const ctl_trunk* h, int n, int hgt, int wid) {
+  int hh = (hgt + 6 - 7) / 2 + 1, ww = (wid + 6 - 7) / 2 + 1;
+  size_t px_ch = (size_t)hh * ww * 64;  // stem conv output
+  hh = (hh + 2 - 3) / 2 + 1;
+  ww = (ww + 2 - 3) / 2 + 1;
+  for (const TrunkBlock& blk : h->blocks) {
+    const int s = blk.c2.stride;
+    const int h2 = (hh + 2 - 3) / s + 1, w2 = (ww + 2 - 3) / s + 1;
+    px_ch = std::max(px_ch, (size_t)hh * ww * blk.c1.cout);
+    px_ch = std::max(px_ch, (size_t)h2 * w2 * std::max(blk.c2.cout, blk.c3.cout));
+    if (blk.has_down) px_ch = std::max(px_ch, (size_t)h2 * w2 * blk.down.cout);
+    hh = h2;
+    ww = w2;
+  }
+  return ((size_t)n * px_ch * 2 + 255) & ~(size_t)255;
 }
 
 size_t ctl_embed_workspace_bytes(const ctl_trunk* h, int32_t n, int32_t hgt, int32_t wid) {
   if (!h || n < 1 || hgt < 8 || wid < 8) return 0;
-  return 5 * trunk_act_bytes(n, hgt, wid);
+  return 5 * trunk_act_bytes(h, n, hgt, wid);
 }
 
 static int run_conv(const PackedConv& c, const void* x, int n, int hh, int ww, const void* residual, void* out, cudaStream_t st) {
@@ -335,7 +351,7 @@ int ctl_embed_forward(ctl_trunk* h, const float* x_nchw, int32_t n, int32_t hgt,
   CTL_CHECK_ARG(h->packed, "ctl_weights_pack has not been called on this handle");
   CTL_CHECK_ARG(n >= 1 && hgt >= 8 && wid >= 8, "bad input shape");
   CTL_CHECK_ARG(out_emb == nullptr || h->has_head, "out_emb needs the bn_head.* tensors in ctl_weights_pack");
-  const size_t act = trunk_act_bytes(n, hgt, wid);
+  const size_t act = trunk_act_bytes(h, n, hgt, wid);
   if (workspace_bytes < 5 * act) {
     set_error("workspace too small: need %zu bytes, have %zu", 5 * act, workspace_bytes);
     return CTL_ERR_WORKSPACE;

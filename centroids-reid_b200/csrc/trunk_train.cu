@@ -387,7 +387,17 @@ static int plan_layout(const ctl_trainer* t, int n, int H, int W, Layout* out) {
   Bump dry;
   Plan plan;
   int rc = forward_walk(&tmp, dry, plan, nullptr, 0, nullptr, n, H, W, nullptr, nullptr);
-  if (!rc) rc = backward_walk(&tmp, dry, plan, nullptr, 0, nullptr, 0, nullptr, 1.f, nullptr);
+  if (rc) return rc;
+  // the backward of a stride-2 layer needs its input map even: the weight gradient (ctl_conv2d_wgrad_nhwc_f16) and the
+  // zero-insertion data gradient (ctl_upsample2_zero_nhwc_f16 writes a [2 ho][2 wo] map) both assume it
+  for (const TrainBlock& b : tmp.blocks)
+    for (const ConvSpec* c : {&b.c1, &b.c2, &b.c3, &b.down})
+      if (c->stride == 2 && (c->h % 2 || c->w_in % 2)) {
+        set_error("%s: a training step needs an even input map at every stride-2 layer, got %dx%d (input %dx%d)",
+                  c->conv.c_str(), c->h, c->w_in, H, W);
+        return CTL_ERR_INVALID_ARGUMENT;
+      }
+  rc = backward_walk(&tmp, dry, plan, nullptr, 0, nullptr, 0, nullptr, 1.f, nullptr);
   if (rc) return rc;
   out->bn_bytes = (plan.bn_need + 255) & ~(size_t)255;
   out->wg_bytes = (plan.wg_need + 255) & ~(size_t)255;
@@ -538,7 +548,10 @@ int ctl_trainer_bind(ctl_trainer* t, const ctl_named_tensor* params, int32_t n_p
 }
 
 size_t ctl_train_workspace_bytes(const ctl_trainer* t, int32_t n, int32_t height, int32_t width) {
-  if (!t || n < 1 || height < 32 || width < 32) return 0;
+  if (!t || n < 1 || height < 32 || width < 32) {
+    set_error("ctl_train_workspace_bytes: bad arguments (n=%d, %dx%d; n >= 1 and sides >= 32 needed)", n, height, width);
+    return 0;
+  }
   Layout l;
   if (plan_layout(t, n, height, width, &l)) return 0;
   return l.total;

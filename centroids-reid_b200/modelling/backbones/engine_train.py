@@ -139,8 +139,22 @@ class TrunkTrainer:
         return z, ho, wo, s
 
     # ---------------------------------------------------------------- forward
+    def check_input_size(self, H: int, W: int):
+        """ValueError unless every stride-2 layer sees an even map at an H x W input: the backward of a stride-2 layer
+        (weight gradient, zero-insertion data gradient) needs it.  Same rule and message as ctl_train_workspace_bytes."""
+        h, w = (H + 6 - 7) // 2 + 1, (W + 6 - 7) // 2 + 1
+        h, w = (h + 2 - 3) // 2 + 1, (w + 2 - 3) // 2 + 1
+        for li in (2, 3, 4) if self.last_stride == 2 else (2, 3):
+            if h % 2 or w % 2:
+                raise ValueError(f"layer{li}.0.conv2: a training step needs an even input map at every stride-2 layer, "
+                                 f"got {h}x{w} (input {H}x{W})")
+            h, w = h // 2, w // 2
+
     def forward(self, x: torch.Tensor, params: Dict[str, torch.Tensor]) -> torch.Tensor:
         """x: [B, 3, H, W] fp32 NCHW on the device -> global_feat [B, 2048] fp32; keeps what backward needs."""
+        if x.dim() != 4:
+            raise ValueError(f"expected [B, 3, H, W], got {tuple(x.shape)}")
+        self.check_input_size(int(x.shape[2]), int(x.shape[3]))
         if not self.graphs:
             return self._forward_impl(x, params)
         N.require_cuda(x)
@@ -407,7 +421,7 @@ class NativeTrainer:
         L = N.lib()
         need = L.ctl_train_workspace_bytes(self._h, n, H, W)
         if need == 0:
-            raise ValueError(f"unsupported input shape {tuple(x.shape)}")
+            raise ValueError(f"unsupported input shape {tuple(x.shape)}: {L.ctl_last_error().decode('utf-8', 'replace')}")
         if self._ws is None or self._ws.numel() < need:
             self._ws = None
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)

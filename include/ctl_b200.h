@@ -236,6 +236,7 @@ int ctl_xent_smooth_step(const float* logits, int32_t b, int32_t c, const int32_
  * modelling/baseline.py:91-96, modelling/bases.py:169-177, inference/inference_utils.py:104-113.
  *   conv2d   : out = [relu]( conv(x, weight) + bias [+ residual] ), weight [Cout][k][k][Cin] fp16
  *              (eval BatchNorm folded in), 1x1 or 3x3 (pad k/2), stride 1 or 2, Cin/Cout % 64 == 0;
+ *              any H, W >= 1 (torch.nn.Conv2d's output size: stride 2 gives ceil(H/2) x ceil(W/2));
  *              ReLU (if relu != 0) is applied to output channels >= relu_from only (IBN: the
  *              InstanceNorm half of bn1 is left raw for ctl_instnorm_relu);
  *   stem     : conv 7x7/2 pad 3 (3 -> 64) + folded BN [+ ReLU] from NCHW fp32 to NHWC fp16;
@@ -296,7 +297,9 @@ int ctl_instnorm_relu_nhwc_f16(void* x, int32_t n, int32_t hw, int32_t c, int32_
  *                        handle.  Call again whenever the parameters change (after opt.step(), load_state_dict).
  *   ctl_embed_forward  : x NCHW fp32 [n][3][h][w] on the device -> out_feat [n][2048] (global_feat) and / or out_emb
  *                        [n][2048] (= eval BatchNorm1d(global_feat); needs the bn_head.* tensors).  Activations live in the
- *                        caller's workspace of ctl_embed_workspace_bytes(...) bytes.  All launches go to `stream`.
+ *                        caller's workspace of ctl_embed_workspace_bytes(...) bytes: five buffers, each the size of the
+ *                        largest activation of the walk (odd sides round up at every stride-2 layer, as in torch).  Any
+ *                        h, w >= 8.  All launches go to `stream`.
  * The handle is per device and not thread-safe; a missing / mis-sized tensor is CTL_ERR_INVALID_ARGUMENT naming it. */
 typedef struct ctl_trunk ctl_trunk;
 typedef struct ctl_named_tensor {
@@ -396,7 +399,9 @@ int ctl_stem_im2col_f16(const float* x_nchw, int32_t n, int32_t h, int32_t w, vo
  *                             torch); `grads` = one fp32 output per PARAMETER, same name, the parameter's own layout
  *                             (conv [Cout][Cin][k][k]).  The handle keeps the pointers: re-bind when storage moves.
  *   ctl_train_workspace_bytes: bytes of the caller's workspace for one (n, h, w) step: the saved activations of the
- *                             forward + the scratch of the backward (≈ 60 MB per 256x128 image).
+ *                             forward + the scratch of the backward (≈ 60 MB per 256x128 image).  0 when the step
+ *                             cannot run: h or w < 32, or an odd map at the input of a stride-2 layer (the backward
+ *                             needs even maps there; ctl_last_error() names the layer and the map size).
  *   ctl_train_forward       : x NCHW fp32 -> out_feat [n][2048] fp32 (global_feat); saved tensors stay in `workspace`.
  *   ctl_train_backward      : dfeat [n][2048] fp32 = dLoss/dglobal_feat.  Activation gradients are computed on
  *                             grad_scale * dfeat in fp16 (loss scaling, the role of PL's GradScaler, utils/misc.py:111);

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- generates tests/golden/*.npz by running the UNMODIFIED
 reference (/root/reference, through oracle/ref_import.py) on seeded synthetic inputs.
 
-    python -m oracle.make_golden [--only loss,retrieval,trunk,trunk_train,trunk_autocast,masks,centroids,market,...]
+    python -m oracle.make_golden [--only loss,retrieval,trunk,trunk_train,trunk_autocast,trunk_geometry,masks,...]
     python -m oracle.make_golden --only ref_cuda_autocast      (on a CUDA device: the reference at the bench shapes)
 
 The reference has no tests and no golden vectors of its own (SURVEY.md section 4); these
@@ -254,6 +254,42 @@ def gen_trunk(ref):
         out[f"{tag}_train_feat"] = gft.numpy()
         print(f"trunk {tag}: feat mean {float(gf.mean()):.5f} std {float(gf.std()):.5f}")
     np.savez_compressed(os.path.join(GOLD, "trunk.npz"), **out)
+
+
+# Eval trunk at input sizes whose feature maps go odd at some stride-2 layer (torch.nn.Conv2d rounds the output up):
+# tag -> (ibn, MODEL.LAST_STRIDE, (H, W)).  tests/test_trunk_geometry_gpu.py sweeps more points; these four are pinned.
+TRUNK_GEOMETRY_CASES = {
+    "r50_s1_300x150": (False, 1, (300, 150)),
+    "r50_s2_260x102": (False, 2, (260, 102)),
+    "ibn_s1_250x125": (True, 1, (250, 125)),
+    "ibn_s2_100x50": (True, 2, (100, 50)),
+}
+
+
+def trunk_geometry_input(ibn, hw, n=3):
+    """Trunk weights and an n-image batch of one geometry point (the golden keeps the first two images)."""
+    return O.make_trunk_state(seed=7, ibn=ibn), torch.randn(n, 3, *hw, generator=torch.Generator().manual_seed(31))
+
+
+def gen_trunk_geometry(ref):
+    """The reference's eval trunk (Baseline, fp32, CPU) at TRUNK_GEOMETRY_CASES: global_feat of two images."""
+    out = {}
+    for tag, (ibn, last_stride, hw) in TRUNK_GEOMETRY_CASES.items():
+        sd, x = trunk_geometry_input(ibn, hw)
+        x = x[:2]
+        cfg = default_cfg(ref)
+        cfg.MODEL.NAME = "resnet50_ibn_a" if ibn else "resnet50"
+        cfg.MODEL.LAST_STRIDE = last_stride
+        base = ref.baseline.Baseline(cfg)
+        base.base.load_state_dict(sd, strict=True)
+        base.eval()
+        with torch.no_grad():
+            _, gf = base(x)
+        out[f"{tag}_in_checksum"] = checksum(x)
+        out[f"{tag}_w_checksum"] = checksum(torch.cat([v.flatten().float() for v in sd.values()]))
+        out[f"{tag}_eval_feat"] = gf.float().numpy()
+        print(f"trunk geometry {tag}: feat mean {float(gf.mean()):.5f} std {float(gf.std()):.5f}")
+    np.savez_compressed(os.path.join(GOLD, "trunk_geometry.npz"), **out)
 
 
 TRAIN_GRAD_KEYS = ("conv1.weight", "bn1.weight", "layer1.0.conv2.weight", "layer1.0.bn1.{bn}weight", "layer2.0.downsample.0.weight",
@@ -509,7 +545,7 @@ def gen_ref_cuda_autocast(ref):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--only", default="loss,loss_variants,masks,retrieval,centroids,trunk,trunk_train,trunk_autocast,market,"
-                                      "triplet_variants,random_erasing")
+                                      "triplet_variants,random_erasing,trunk_geometry")
     args = ap.parse_args()
     only = set(args.only.split(","))
     os.makedirs(GOLD, exist_ok=True)
@@ -540,6 +576,8 @@ def main():
         gen_triplet_variants(ref)
     if "random_erasing" in only:
         gen_random_erasing(ref)
+    if "trunk_geometry" in only:
+        gen_trunk_geometry(ref)
     if "ref_cuda_autocast" in only:  # needs a CUDA device; not in the default list
         gen_ref_cuda_autocast(ref)
 

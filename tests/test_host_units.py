@@ -92,7 +92,7 @@ def test_c_abi_argument_errors_are_reported_without_a_gpu():
     cases = [
         lambda: L.ctl_conv2d_nhwc_f16(one, 1, 8, 8, 48, one, one, None, one, 64, 1, 1, 0, 0, None),          # Cin % 64
         lambda: L.ctl_conv2d_nhwc_f16(one, 1, 8, 8, 64, one, one, None, one, 64, 5, 1, 0, 0, None),          # 5x5
-        lambda: L.ctl_conv2d_nhwc_f16(one, 1, 7, 8, 64, one, one, None, one, 64, 3, 2, 0, 0, None),          # odd H, stride 2
+        lambda: L.ctl_conv2d_nhwc_f16(one, 1, 7, 8, 64, one, one, None, one, 64, 3, 3, 0, 0, None),          # stride 3
         lambda: L.ctl_conv2d_wgrad_nhwc_f16(one, 1, 8, 8, 64, one, 96, 1, 1, one, 1 << 30, one, None),       # Cout % 64
         lambda: L.ctl_bn_train_forward_nhwc_f16(one, 10, 48, 48, one, one, 1e-5, 0.1, None, None, None, 0, one, 1 << 20,
                                                  one, one, one, None),                                         # C not a power of two
@@ -169,3 +169,86 @@ def test_identity_orders_and_encoded_ids_on_the_host():
         return np.mean([not (b[1] < a[0] or b[0] > a[1]) for a in qr for b in gr])
     assert hot_fraction(srt.q_pid.numpy(), srt.g_pid.numpy()) < 0.5 < hot_fraction(plain.q_pid.numpy(), plain.g_pid.numpy())
     assert not R.pid_order_pays(3368, 15913) and R.pid_order_pays(50000, 25000)
+
+
+def _trunk_walk(H, W, last_stride):
+    """Layer walk of the eval trunk at an H x W input with torch.nn.Conv2d / MaxPool2d output sizes (elementwise over numpy
+    arrays H, W): (elements of the largest activation per image -- stem conv, max-pool and every conv output --, and the
+    input map (h, w) of every stride-2 bottleneck layer as (name, h, w))."""
+    h, w = (H + 6 - 7) // 2 + 1, (W + 6 - 7) // 2 + 1
+    big = h * w * 64
+    h, w = (h + 2 - 3) // 2 + 1, (w + 2 - 3) // 2 + 1
+    big = np.maximum(big, h * w * 64)
+    strided = []
+    for li, (planes, nblk) in enumerate(zip((64, 128, 256, 512), (3, 4, 6, 3)), start=1):
+        for bi in range(nblk):
+            s = (1 if li == 1 else (last_stride if li == 4 else 2)) if bi == 0 else 1
+            if s == 2:
+                strided.append((f"layer{li}.{bi}.conv2", h, w))
+            h2, w2 = (h - 1) // s + 1, (w - 1) // s + 1
+            big = np.maximum(big, h * w * planes)            # conv1
+            big = np.maximum(big, h2 * w2 * planes * 4)      # conv3 / downsample (conv2 is smaller)
+            h, w = h2, w2
+    return big, strided
+
+
+def test_embed_workspace_covers_the_largest_activation_at_every_input_size():
+    """ctl_embed_forward ping-pongs five buffers of ctl_embed_workspace_bytes / 5 bytes, so each must hold the largest
+    activation of the walk.  When the stem output has an odd side the max-pool rounds up, and layer1's output
+    [n, ceil(h/2), ceil(w/2), 256] outgrows the stem's conv output; at tiny inputs the 2048-channel maps do."""
+    import ctypes as C
+
+    from ctl_b200 import _native as N
+
+    L = N.lib()
+    sides = np.arange(8, 401)
+    H, W = np.meshgrid(sides, sides, indexing="ij")
+    H, W = H.ravel(), W.ravel()
+    for ibn in (0, 1):
+        for last_stride in (1, 2):
+            h = C.c_void_p()
+            assert L.ctl_trunk_create(C.byref(h), ibn, last_stride) == 0
+            try:
+                got = np.array([L.ctl_embed_workspace_bytes(h, 1, int(a), int(b)) for a, b in zip(H, W)], dtype=np.int64)
+                got3 = L.ctl_embed_workspace_bytes(h, 3, 300, 150)
+            finally:
+                L.ctl_trunk_destroy(h)
+            need = 5 * 2 * _trunk_walk(H, W, last_stride)[0]
+            bad = np.nonzero(got < need)[0]
+            assert bad.size == 0, (
+                f"ibn={ibn} last_stride={last_stride}: {bad.size} sizes under-sized, e.g. " +
+                ", ".join(f"{H[i]}x{W[i]}: {got[i] // 5} bytes per buffer < {need[i] // 5}" for i in bad[:5]))
+            assert got3 >= 3 * 5 * 2 * int(_trunk_walk(300, 150, last_stride)[0])  # the buffers scale with the batch
+
+
+def test_train_workspace_rejects_exactly_the_sizes_training_cannot_run():
+    """A training step needs an even input map at every stride-2 layer (weight gradient and zero-insertion data
+    gradient); ctl_train_workspace_bytes is 0 for exactly the other sizes, and ctl_last_error() names the first such
+    layer and its map size."""
+    import ctypes as C
+
+    from ctl_b200 import _native as N
+
+    L = N.lib()
+    sides = np.r_[32:80, 96, 126, 127, 128, 150, 160, 250, 256, 300, 320, 384, 400]
+    for ibn in (0, 1):
+        for last_stride in (1, 2):
+            h = C.c_void_p()
+            assert L.ctl_trainer_create(C.byref(h), ibn, last_stride, 0.1) == 0
+            try:
+                for H in sides:
+                    for W in sides:
+                        odd = [(name, a, b) for name, a, b in _trunk_walk(int(H), int(W), last_stride)[1] if a % 2 or b % 2]
+                        got = L.ctl_train_workspace_bytes(h, 2, int(H), int(W))
+                        assert (got == 0) == bool(odd), (ibn, last_stride, H, W, got, odd)
+                        if odd:
+                            msg = L.ctl_last_error().decode()
+                            name, a, b = odd[0]
+                            assert name in msg and f"{a}x{b}" in msg, (H, W, msg)
+            finally:
+                L.ctl_trainer_destroy(h)
+            # 300x150: layer1 leaves a 75x38 map, which layer2.0 would subsample
+            assert L.ctl_trainer_create(C.byref(h), ibn, last_stride, 0.1) == 0
+            assert L.ctl_train_workspace_bytes(h, 4, 300, 150) == 0
+            assert b"layer2.0.conv2" in L.ctl_last_error() and b"75x38" in L.ctl_last_error()
+            L.ctl_trainer_destroy(h)

@@ -500,3 +500,27 @@ def test_native_trainer_argument_errors():
     assert rc != 0 and b"workspace of the forward" in N.lib().ctl_last_error()
     tr.backward(df)  # the right workspace still works
     torch.cuda.synchronize()
+
+
+@pytest.mark.parametrize("which", ["python", "python_graphs", "native"])
+def test_trainers_reject_odd_stride2_maps_before_any_launch(which):
+    """A training step cannot run where a stride-2 layer would see an odd map (300x150: layer1 leaves 75x38).  Both
+    trainers raise ValueError naming the layer and the map size before anything runs on the device: the BatchNorm
+    running statistics they were given are unchanged."""
+    from oracle import ctl_oracle as O
+    from ctl_b200.modelling.backbones.engine_train import NativeTrainer, TrunkTrainer
+
+    sd = O.make_trunk_state(seed=3)
+    params = {k: v.clone().cuda().contiguous() for k, v in sd.items() if v.is_floating_point()}
+    running = {k: v.clone() for k, v in params.items() if "running" in k}
+    x = torch.randn(2, 3, 300, 150, generator=torch.Generator().manual_seed(1)).cuda()
+    if which == "native":
+        tr = NativeTrainer(params, "cuda:0")
+        call = lambda: tr.forward(x)  # noqa: E731
+    else:
+        tr = TrunkTrainer("cuda:0", graphs=which == "python_graphs")
+        call = lambda: tr.forward(x, params)  # noqa: E731
+    with pytest.raises(ValueError, match=r"layer2\.0\.conv2.*75x38"):
+        call()
+    torch.cuda.synchronize()
+    assert all(torch.equal(params[k], v) for k, v in running.items())

@@ -66,6 +66,20 @@ def _conv_case(n, h, w, cin, cout, k, stride, relu, residual, relu_from=0, seed=
     (1, 80, 80, 64, 64, 3, 1, True, False),
     (2, 40, 40, 128, 128, 3, 2, True, False),
     (1, 7, 5, 64, 128, 3, 1, False, True),        # tiny, heavily over-covered tile
+    # stride 2 on odd sides: the odd parity view is one pixel shorter, its zero-fill is the bottom / right padding
+    (3, 75, 38, 64, 128, 3, 2, True, False),      # layer2.0 conv2 at 300x150; 128-wide tiles
+    (2, 38, 19, 128, 256, 3, 2, True, False),
+    (4, 19, 10, 256, 512, 3, 2, True, True),      # residual
+    (3, 75, 38, 256, 512, 1, 2, False, False),    # layer2.0 downsample at 300x150
+    (2, 13, 7, 1024, 2048, 1, 2, False, True),    # layer4.0 downsample at 208x104, LAST_STRIDE 2; residual
+    (2, 7, 7, 64, 64, 3, 2, True, False),         # 64-wide tiles
+    (3, 9, 5, 256, 256, 3, 2, False, False),
+    # one-pixel sides at stride 2: the odd parity views are empty and their taps are dropped
+    (2, 1, 1, 256, 256, 3, 2, True, False),
+    (2, 1, 5, 256, 256, 3, 2, True, False),
+    (2, 5, 1, 128, 256, 3, 2, False, True),
+    (2, 1, 1, 1024, 2048, 1, 2, False, False),
+    (3, 1, 7, 128, 128, 1, 2, True, False),
 ])
 def test_conv_shapes(case):
     _conv_case(*case)
@@ -181,6 +195,63 @@ def test_stem_maxpool_gap_instnorm():
     got = td.cpu()
     assert torch.equal(got[..., 64:], t[..., 64:])
     assert float((got[..., :64].double() - ref_in).abs().max()) <= float(ref_in.abs().max()) * 2.0 ** -10 + 2e-3
+
+
+@pytest.mark.parametrize("path,shape", [
+    ("tc", (2, 250, 125)),     # stem output 125x63, pooled 63x32
+    ("tc", (3, 97, 33)),       # 49x17 -> 25x9
+    ("tc", (2, 9, 8)),         # 5x4 -> 3x2
+    ("fused", (2, 260, 102)),  # 130x51 -> 65x26
+    ("fused", (3, 8, 128)),    # 4x64 -> 2x32
+    ("fused", (2, 12, 126)),   # 6x63 -> 3x32
+])
+def test_stem_at_odd_sizes(path, shape):
+    """The stem where its conv output or the pooled map has an odd side (the max-pool rounds up, its last window is
+    clipped).  `tc`: ctl_stem_conv7x7_tc against the float64 convolution of the same fp16 operands, then
+    ctl_maxpool3x3s2_nhwc_f16 EXACTLY equal to F.max_pool2d of the kernel's own stem output.  `fused`:
+    ctl_stem_pool_fused against the float64 convolution followed by max_pool2d."""
+    from ctl_b200 import _native as N
+    from ctl_b200.modelling.backbones.engine import pack_stem_fused
+
+    L = N.lib()
+    n, H, W = shape
+    g = torch.Generator().manual_seed(H * 1000 + W)
+    x = torch.randn(n, 3, H, W, generator=g)
+    w = torch.randn(64, 3, 7, 7, generator=g) * 0.1
+    b = torch.randn(64, generator=g) * 0.1
+    xd, bd = x.cuda(), b.cuda()
+    for relu in (0, 1):
+        ref = F.conv2d(x.half().double(), w.half().double(), b.double(), 2, 3)
+        if relu:
+            ref = ref.clamp(min=0)
+        refp = F.max_pool2d(ref, 3, 2, 1)
+        ho, wo = ref.shape[2:]
+        hp, wp = refp.shape[2:]
+        if path == "tc":
+            wk192 = torch.zeros(64, 21, 8)
+            wk192[:, :, :7] = w.reshape(64, 21, 7)
+            wk192 = torch.cat((wk192.reshape(64, 168), torch.zeros(64, 24)), 1).half().cuda()
+            s = torch.full((n, ho, wo, 64), float("nan"), dtype=torch.float16, device="cuda")
+            N.check(L.ctl_stem_conv7x7_tc(xd.data_ptr(), n, H, W, wk192.data_ptr(), bd.data_ptr(), relu, s.data_ptr(),
+                                          N.stream_ptr()))
+            torch.cuda.synchronize()
+            got = s.cpu().double().permute(0, 3, 1, 2)
+            assert torch.isfinite(got).all()
+            assert float((got - ref).abs().max()) <= float(ref.abs().max()) * 2.0 ** -10 + 1e-4
+            pooled = torch.full((n, hp, wp, 64), float("nan"), dtype=torch.float16, device="cuda")
+            N.check(L.ctl_maxpool3x3s2_nhwc_f16(s.data_ptr(), n, ho, wo, 64, pooled.data_ptr(), N.stream_ptr()))
+            refs = F.max_pool2d(s.cpu().float().permute(0, 3, 1, 2), 3, 2, 1).permute(0, 2, 3, 1)
+            assert torch.equal(pooled.cpu().float(), refs)
+        else:
+            wd = pack_stem_fused(w.cuda())
+            pad = torch.zeros(L.ctl_stem_pad_bytes(n, H, W), dtype=torch.uint8, device="cuda")
+            out = torch.full((n, hp, wp, 64), float("nan"), dtype=torch.float16, device="cuda")
+            N.check(L.ctl_stem_pool_fused(xd.data_ptr(), n, H, W, pad.data_ptr(), wd.data_ptr(), bd.data_ptr(), relu,
+                                          out.data_ptr(), N.stream_ptr()))
+            torch.cuda.synchronize()
+            got = out.cpu().double().permute(0, 3, 1, 2)
+            assert torch.isfinite(got).all()
+            assert float((got - refp).abs().max()) <= float(refp.abs().max()) * 2.0 ** -10 + 1e-4
 
 
 @pytest.mark.parametrize("tag,ibn,hw", [("r50", False, (256, 128)), ("ibn", True, (128, 64))])
